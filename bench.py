@@ -326,6 +326,28 @@ class Workload:
         return int(np.prod(self.out_shape)) * 4 + self.batch * 4
 
 
+DUMP_BYTES = 60 * 10**6  # the .npy headers on top stay far inside 64 MB
+
+
+def dump_outputs(wl, out_dir):
+    """--dump-outputs: what the last timed step computed, as a caller of the device-resident path receives it - every model
+    output (for a detector, the head tensors its YOLO layer reads), float32 NHWC - written as out_dir/<name>.npy. Outputs
+    that together exceed 60 MB are each cut to the same fixed, seeded sample of their flattened elements (ascending index)."""
+    m = wl.model
+    if wl.detector:
+        yi = [i for i, l in enumerate(wl.layers) if l["type"] == "YOLO"][0]
+        arrays = {"yolo_head_%d" % k: m.layer_output(j) for k, j in enumerate(wl.layers[yi]["inputId"])}
+    else:
+        arrays = {"output_%d" % i: m.get_output(i) for i in range(m.num_outputs)}
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if total > DUMP_BYTES:
+            a = a.ravel()
+            a = a[np.unique(np.random.default_rng(0).integers(0, a.size, a.size * DUMP_BYTES // total))]
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
+
+
 def kernel_roofline(wl, work, pk, terms, step_ms, reps=5):
     """Per-layer event pairs (eager pass, live) -> per-kernel totals; the DOMINANT kernel's algorithmic bytes / flops over its own
     event time against the bound that binds IT. Also the per-layer table rows."""
@@ -437,7 +459,10 @@ def main():
     ap.add_argument("--precision", default="fp32x3", choices=["fp32x3", "fp16w", "fp16"],
                     help="product form of the tensor-core path (snnb.h SNNB_PRECISION_*); the headline is fp32x3")
     ap.add_argument("--batch", type=int, default=0, help="override the workload's batch per GPU (the metric's config is the default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step (rank 0) as DIR/<name>.npy, float32, 64 MB at most")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
 
     from shadernn_b200 import parallel
@@ -479,6 +504,8 @@ def main():
         wl.ctx.sync()
     dev_ms, launches, region = wl.device_loop(args.steps, args.warmup, lib, check)
     clocks = sampler.stop(region)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(wl, args.dump_outputs)
 
     # ---- end to end through the C-ABI with host buffers ("e2e") ----
     u8_ms = wl.e2e_loop(args.steps, True)

@@ -1,8 +1,9 @@
-"""Generate tests/golden/ref_cpu_golden.npz from the REFERENCE ITSELF (oracle/_ref/libsnn_ref.so = the reference's
-core/src/ic2/cpulayer.h + demo/common/prng.h compiled where they lie under /root/reference).
+"""Generate tests/golden/ref_cpu_golden.npz and tests/golden/ref_cpu_live_golden.npz from the REFERENCE ITSELF
+(oracle/_ref/libsnn_ref.so = the reference's core/src/ic2/cpulayer.h + demo/common/prng.h, compiled where they lie in a
+reference checkout).
 
-/root/reference does not exist on the GPU box, so the outputs are committed here as a small fixture and this script is
-the recipe that produced them:   make -C oracle ref && python tests/golden/make_golden.py
+The reference is not part of this repository, so its outputs are committed here as small fixtures and this script is the
+recipe that produced them:   make -C oracle ref REF=<reference checkout> && python tests/golden/make_golden.py
 """
 import ctypes as C
 import os
@@ -60,5 +61,29 @@ def main():
     print("wrote", path, "smoke softmax:", y)
 
 
+def live_cases():
+    """The long PRNG streams and the Dense cases that tests/test_oracle_cpu.py holds the oracle to (the *_live_reference tests)."""
+    r = oracle.ref()
+    assert r is not None, "build oracle/_ref first (needs a reference checkout)"
+    out = {}
+    for seed in (7767517, 1, 123456789):
+        r.ref_srand(C.c_uint64(seed))
+        out["prng_u64_%d" % seed] = np.array([r.ref_rand_u64() for _ in range(3000)], dtype=np.uint64)  # crosses several 55-draw refills
+    rng = np.random.default_rng(5)
+    for act in ["", "relu", "leakyRelu", "sigmoid", "tanh", "softmax"]:
+        x = rng.uniform(-2, 2, 37).astype(np.float32)
+        k = rng.uniform(-1, 1, (9, 37)).astype(np.float32)
+        b = rng.uniform(-1, 1, 9).astype(np.float32)
+        y = np.empty(9, np.float32)
+        assert r.ref_dense(x.ctypes.data_as(C.c_void_p), 37, k.ctypes.data_as(C.c_void_p), b.ctypes.data_as(C.c_void_p), 9, act.encode(), 0.2,
+                           y.ctypes.data_as(C.c_void_p)) == 0
+        for s, v in zip("xkby", (x, k, b, y)):
+            out["dense_%s_%s" % (act or "linear", s)] = v
+    path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "ref_cpu_live_golden.npz")
+    np.savez_compressed(path, **out)
+    print("wrote", path)
+
+
 if __name__ == "__main__":
     main()
+    live_cases()

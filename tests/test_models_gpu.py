@@ -301,18 +301,24 @@ def test_real_candy_weights_head_vs_torch_golden(ctx, tmp_path, precision):
     assert rel < LIMIT[precision]
 
 
-REF_MODELS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "_ref_models")
+@pytest.fixture(scope="module")
+def candy_whole(tmp_path_factory):
+    # the reference's whole candy-9_simplified.onnx as tests/_candy_fixture.py writes it (its graph, its 1-D initialisers,
+    # seeded convolution kernels), converted at 224x224, and torch's evaluation of that ONNX graph
+    from _candy_fixture import whole_model_onnx
+    from shadernn_b200 import onnx2snn
+    d = tmp_path_factory.mktemp("candy_whole")
+    src = whole_model_onnx(str(d / "candy-9_simplified.onnx"))
+    path, _ = onnx2snn.convert(src, str(d), input_hw=(224, 224))
+    x = modelzoo.synthetic_input("candy", 1, (224, 224))
+    return path, x, onnx2snn.torch_eval(onnx2snn.load_onnx(src), x)
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF_MODELS, "candy-9_simplified_layers.json")),
-                    reason="tests/golden/_ref_models/ is generated by __graft_entry__.build() where /root/reference exists (and travels with the snapshot)")
 @pytest.mark.parametrize("precision", ["fp32x3", "fp16w"])
-def test_real_candy_whole_model_vs_torch_and_oracle(ctx, precision):
-    # the WHOLE real-weight model (converted from the reference's ONNX file by build()): final image against torch's evaluation
-    # of the ONNX graph (golden, generated with it) and every layer against the oracle
-    path = os.path.join(REF_MODELS, "candy-9_simplified_layers.json")
-    z = np.load(os.path.join(REF_MODELS, "candy_full_golden.npz"))
-    x, want = z["x"], z["y"]
+def test_real_candy_whole_model_vs_torch_and_oracle(ctx, candy_whole, precision):
+    # the WHOLE model converted from the reference's ONNX file: final image against torch's evaluation of the ONNX graph and
+    # every layer against the oracle
+    path, x, want = candy_whole
     layers_want = oracle.Model(path).run(x, return_all=True)
     m = core.MixedInferenceCore(ctx, path, batch=1, fuse=False, precision=precision)
     m.set_input(x)

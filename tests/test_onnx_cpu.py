@@ -1,35 +1,24 @@
 """ONNX -> ShaderNN JSON converter (shadernn_b200/onnx2snn.py, SURVEY §8 f-N1): the hand-rolled protobuf reader, the
-conversion rules, and — the one reference-held pin the conv path has — the real weights of
-modelzoo/StyleTransfer/candy-9_simplified.onnx: the converted model, walked by the oracle, must reproduce what torch computes
-for the ONNX graph itself. The committed fixture (tests/golden/candy_head_golden.npz, generator beside it) carries the first
-two stages' initialisers and torch's outputs, so the check also runs where /root/reference does not exist."""
+conversion rules, and — the one reference-held pin the conv path has — modelzoo/StyleTransfer/candy-9_simplified.onnx: the
+converted model, walked by the oracle, must reproduce what torch computes for the ONNX graph itself. Two committed fixtures
+(generator tests/golden/make_candy_golden.py) stand in for the 6.7 MB file: candy_head_golden.npz carries the first two
+stages' real initialisers and torch's outputs; candy_graph_golden.npz the whole file except the convolution kernels' values."""
 import os
 import struct
 
 import numpy as np
-import pytest
 
 from oracle import oracle
 from shadernn_b200 import modelzoo, onnx2snn
 
 from _candy_fixture import head_graph as _head_graph
+from _candy_fixture import varint as _vi
+from _candy_fixture import whole_model_onnx
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF_ONNX = "/root/reference/modelzoo/StyleTransfer/candy-9_simplified.onnx"
 
 
 # ---- a minimal protobuf ENCODER, test-side only, to feed the reader with hand-made messages -------------------------
-def _vi(v):
-    out = b""
-    v &= (1 << 64) - 1
-    while True:
-        b = v & 0x7F
-        v >>= 7
-        out += bytes([b | (0x80 if v else 0)])
-        if not v:
-            return out
-
-
 def _ld(field, payload):
     return _vi((field << 3) | 2) + _vi(len(payload)) + payload
 
@@ -119,11 +108,12 @@ def test_real_candy_weights_head_matches_torch_golden(tmp_path):
     assert float(np.abs(got - want).max()) <= 5e-5 * float(np.abs(want).max())
 
 
-@pytest.mark.skipif(not os.path.exists(REF_ONNX), reason="the reference checkout (candy-9_simplified.onnx) is not on this machine")
 def test_whole_candy_model_from_the_reference_checkout(tmp_path):
-    g = onnx2snn.load_onnx(REF_ONNX)
+    # the reference's file as the fixture holds it: its own graph and encoding, seeded convolution kernels (_candy_fixture)
+    src = whole_model_onnx(str(tmp_path / "candy-9_simplified.onnx"))
+    g = onnx2snn.load_onnx(src)
     assert len(g["nodes"]) == 64 and len(g["init"]) == 64
-    path, layers = onnx2snn.convert(REF_ONNX, str(tmp_path), input_hw=(96, 96))
+    path, layers = onnx2snn.convert(src, str(tmp_path), input_hw=(96, 96))
     assert os.path.basename(path) == "candy-9_simplified_layers.json" and os.path.exists(str(tmp_path / "candy-9_simplified_weights.bin"))  # onnxToJsonConverter.py:69-73
     assert len(layers) == 39 and sum(l["type"] == "Conv2D" for l in layers) == 16 and sum(l["type"] == "InstanceNormalization" for l in layers) == 15
     x = modelzoo.synthetic_input("candy", 1, (96, 96))
