@@ -290,6 +290,11 @@ int snnb_debug_streamk_schedule(int tiles, int num_kb, int sms, int* rows, int c
  * ksteps (K = 16 steps per filter row), rows_per_panel (filter rows sharing one 128-byte weight row)}. Returns 1 if the layer can use
  * the feed mode, 0 if not. No GPU needed. */
 int snnb_debug_feed_plan(int k, int stride, int pad_x, int ic, int out[5]);
+/* Diagnostics: every K block the tensor-core producer loads for a `ksize` x `ksize` convolution over `cblocks` 64-channel blocks (channel
+ * pitch `icp`) with a folded 1x1 shortcut of `sc_cblocks` channel blocks (0: none), for `tiles` output tiles split into `ksplit` K ranges
+ * (0: stream-K over `sms` SMs). rows = capacity x 6 ints {tile, kb, shortcut, tap, channel block, weight column}, in each work item's
+ * order; returns the number of rows (may exceed capacity), -1 for invalid arguments or nothing to cut (stream-K). No GPU needed. */
+int snnb_debug_kblock_schedule(int ksize, int cblocks, int icp, int sc_cblocks, int tiles, int ksplit, int sms, int* rows, int capacity);
 
 #ifdef __cplusplus
 }

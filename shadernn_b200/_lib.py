@@ -144,6 +144,7 @@ SIGNATURES = {
     "snnb_tensor_planes": (C.c_int, [vp, C.POINTER(vp), C.POINTER(vp), c_int_p]),
     "snnb_debug_streamk_schedule": (C.c_int, [C.c_int, C.c_int, C.c_int, c_int_p, C.c_int]),
     "snnb_debug_feed_plan": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, c_int_p]),
+    "snnb_debug_kblock_schedule": (C.c_int, [C.c_int] * 7 + [c_int_p, C.c_int]),
 }
 
 _lib = None

@@ -150,6 +150,10 @@ int snnb_debug_streamk_schedule(int tiles, int num_kb, int sms, int* rows, int c
     SNNB_REQUIRE(rows || capacity == 0, "snnb_debug_streamk_schedule: null buffer");
     return streamk_schedule(tiles, num_kb, sms, rows, capacity);
 }
+int snnb_debug_kblock_schedule(int ksize, int cblocks, int icp, int sc_cblocks, int tiles, int ksplit, int sms, int* rows, int capacity) {
+    SNNB_REQUIRE(rows || capacity == 0, "snnb_debug_kblock_schedule: null buffer");
+    return kblock_schedule(ksize, cblocks, icp, sc_cblocks, tiles, ksplit, sms, rows, capacity);
+}
 int snnb_tensor_planes(const snnb_tensor* t, void** hi, void** lo, int* cp) {
     SNNB_REQUIRE(t && hi && lo && cp, "snnb_tensor_planes: null argument");
     *hi = t->hi, *lo = t->lo, *cp = t->cp;

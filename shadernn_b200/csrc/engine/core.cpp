@@ -88,6 +88,46 @@ bool MixedInferenceCore::init(std::string& err) {
     // ---- fusion passes (engine-level; off => one kernel per reference layer, every layer output observable) ----
     // `alias[L]` = the layer whose output tensor stands in for L's (L launches nothing).
     std::unordered_map<GenericModelLayer*, GenericModelLayer*> alias;
+    // SNNB_NO_SHORTCUT_FOLD: profiling switch, read at every load so that one process can compare both forms
+    const bool shortcutFold = options.fuse && options.convAlgo != SNNB_ALGO_SIMT && getenv("SNNB_NO_SHORTCUT_FOLD") == nullptr;
+    // Can `c2` (k x k, stride 1) take the 1x1 projection `ds` of another tensor as extra K blocks? Shapes, order and the tensor-core
+    // planner decide (conv2d_umma_fold_supported, asked with stand-in tensors of the planned shapes: nothing is allocated yet).
+    auto foldable = [&](GenericModelLayer* c2, GenericModelLayer* ds) {
+        if (c2 == ds || c2->typeName != "Conv2D" || ds->typeName != "Conv2D" || c2->fusedAway || ds->fusedAway) return false;
+        auto* cc = static_cast<Conv2DLayer*>(c2);
+        auto* dc = static_cast<Conv2DLayer*>(ds);
+        if (c2->nextLayers.size() != 1 || ds->nextLayers.size() != 1 || c2->prevLayers.size() != 1 || ds->prevLayers.size() != 1) return false;
+        if (cc->_desc.activation.id != SNNB_ACT_NONE || dc->_desc.activation.id != SNNB_ACT_NONE || cc->residual || cc->fusedAct >= 0 || cc->shortcut ||
+            dc->shortcut || dc->foldedInto)
+            return false;
+        // a 1x1 convolution runs with pad 0 whatever its padding spec says (Conv2DLayer::run): the fold reads what its own launch reads
+        const int dsMode = padModeId(dc->_desc.padding.mode);
+        if (cc->_desc.stride != 1 || dc->_desc.kernelSize != 1 || !(dsMode == SNNB_PAD_NONE || dsMode == SNNB_PAD_CONSTANT)) return false;
+        GenericModelLayer* x = ds->prevLayers[0];
+        if (order[x] >= order[c2]) return false; // the shortcut's input must be complete when c2 runs
+        const Dims &dc2 = graph.outputDims[order[c2]], &dds = graph.outputDims[order[ds]];
+        if (dc2.width != dds.width || dc2.height != dds.height || dc2.depth != dds.depth || graph.outputDims[order[x]].depth != ds->numInputPlanes) return false;
+        auto stand_in = [&](GenericModelLayer* X) {
+            snnb_tensor t;
+            const Dims& d = graph.outputDims[order[X]];
+            t.n = N, t.h = (int) d.height, t.w = (int) d.width, t.c = (int) d.depth, t.cp = round_up(t.c, 8);
+            t.hi = reinterpret_cast<__half*>(1), t.lo = twoPlanes ? t.hi : nullptr;
+            return t;
+        };
+        const snnb_tensor in = stand_in(c2->prevLayers[0]), sc = stand_in(x), out = stand_in(c2);
+        snnb_weights probe; // "tensor path available", with the row-window operand the layer would be packed with (as wantsPrepad asks)
+        probe.w_hi = probe.w_lo = probe.w_row_hi = probe.w_row_lo = reinterpret_cast<__half*>(1);
+        uint32_t offs[4];
+        cc->_desc.padding.offsets((int) cc->_desc.kernelSize, true, offs);
+        ConvArgs a;
+        a.in = &in, a.residual = nullptr, a.out = const_cast<snnb_tensor*>(&out), a.w = &probe;
+        a.k = (int) cc->_desc.kernelSize, a.stride = 1;
+        a.pad_x = a.k == 1 ? 0 : (int) offs[0], a.pad_y = a.k == 1 ? 0 : (int) offs[2], a.pad_mode = padModeId(cc->_desc.padding.mode);
+        probe.row_stride = 1, probe.row_pad = a.pad_x;
+        a.act = SNNB_ACT_NONE, a.alpha = 0.0f, a.precision = options.precision;
+        a.shortcut = &sc, a.sc_stride = (int) dc->_desc.stride;
+        return conv2d_umma_fold_supported(ctx, a);
+    };
     if (options.fuse) {
         for (auto* L : graph.sorted) {
             // (1) Pad -> Conv2D/Depthwise with zero own padding: the consumer's gather applies the offsets (and mode) itself.
@@ -106,8 +146,29 @@ bool MixedInferenceCore::init(std::string& err) {
                     alias[L]       = L->prevLayers[0];
                 }
             }
+            // (5) Conv2D(k x k, stride 1) + Conv2D(1x1 projection of another tensor) -> Add(+act), as in a down-sampling ResNet block:
+            // Add(c2(y), ds(x)) = [W2 | Wds] . [im2col(y) ; x_strided] + (b2 + bds), one GEMM whose K loop runs on into the projection's
+            // channels. c2 writes the Add's tensor with the Add's activation; ds and the Add launch nothing, and ds has no tensor.
+            // Where it cannot fire, (2) fuses the Add into one of the convs as before.
+            if (shortcutFold && L->typeName == "Add" && L->prevLayers.size() == 2) {
+                auto* add = static_cast<AddLayer*>(L);
+                for (int o = 0; o < 2; ++o) {
+                    GenericModelLayer* c2 = L->prevLayers[o];
+                    GenericModelLayer* ds = L->prevLayers[1 - o];
+                    if (!foldable(c2, ds)) continue;
+                    auto* cc       = static_cast<Conv2DLayer*>(c2);
+                    cc->fusedAct   = add->activation.id;
+                    cc->fusedAlpha = add->activation.alpha;
+                    cc->shortcut   = static_cast<Conv2DLayer*>(ds);
+                    cc->shortcut->foldedInto = cc;
+                    ds->fusedAway  = true;
+                    L->fusedAway   = true;
+                    alias[c2]      = L; // c2 output == add output
+                    break;
+                }
+            }
             // (2) Conv2D(linear) -> Add(+act): the conv's epilogue adds the other operand and applies the Add's activation.
-            if (L->typeName == "Add" && L->prevLayers.size() == 2) {
+            if (L->typeName == "Add" && L->prevLayers.size() == 2 && !L->fusedAway) {
                 auto* add = static_cast<AddLayer*>(L);
                 GenericModelLayer* a = L->prevLayers[0];
                 GenericModelLayer* b = L->prevLayers[1];
@@ -172,6 +233,7 @@ bool MixedInferenceCore::init(std::string& err) {
         if (L->typeName == "YOLO") continue; // host op
         GenericModelLayer* owner = resolve(L);
         if (owner != L && !(L->typeName == "Conv2D")) continue; // Pad/Flatten aliases own nothing
+        if (L->typeName == "Conv2D" && static_cast<Conv2DLayer*>(L)->foldedInto) continue; // a folded shortcut writes nothing
         if (outOf.count(owner)) continue;
         // dims of the tensor = dims of `owner` (for conv->add fusion both agree)
         const Dims& d = graph.outputDims[order[owner]];
@@ -192,7 +254,7 @@ bool MixedInferenceCore::init(std::string& err) {
         L->output                = outOf.count(owner) ? outOf[owner] : nullptr;
         if (L->fusedAway) continue;
         size_t nin = L->prevLayers.size();
-        if (L->typeName == "Conv2D" && static_cast<Conv2DLayer*>(L)->fusedAct >= 0) {
+        if (L->typeName == "Conv2D" && static_cast<Conv2DLayer*>(L)->fusedAct >= 0 && !static_cast<Conv2DLayer*>(L)->shortcut) {
             nin -= 1; // last prev is the residual operand
             L->residual = outOf.at(resolve(L->prevLayers.back()));
         }
@@ -200,6 +262,7 @@ bool MixedInferenceCore::init(std::string& err) {
         if (L->typeName == "Conv2D") {
             auto* cl  = static_cast<Conv2DLayer*>(L);
             cl->algo = options.convAlgo;
+            if (cl->shortcut) cl->shortcutIn = outOf.at(resolve(cl->shortcut->prevLayers[0]));
             // weights are not packed yet: probe with a weights stub that says "tensor path available"
             int ph = 0, pw = 0;
             snnb_weights probe_w;
@@ -227,7 +290,7 @@ bool MixedInferenceCore::init(std::string& err) {
                 cl->_desc.padding.offsets((int) cl->_desc.kernelSize, true, offs);
                 const int k = (int) cl->_desc.kernelSize, padX = (int) offs[0], padY = (int) offs[2];
                 FeedPlan fp;
-                if (!noFeed && !prepad && src->isInputLayer && !in->feed_hi && options.convAlgo != SNNB_ALGO_SIMT && !L->residual && L->output->c <= 64 &&
+                if (!noFeed && !prepad && src->isInputLayer && !in->feed_hi && options.convAlgo != SNNB_ALGO_SIMT && !L->residual && !cl->shortcut && L->output->c <= 64 &&
                     (mode == SNNB_PAD_NONE || mode == SNNB_PAD_CONSTANT) && make_feed_plan(k, (int) cl->_desc.stride, padX, in->c, fp)) {
                     const int tilesX = (L->output->w + 127) / 128;
                     const int needW  = 2 * (tilesX * 128 - 1) + 2 * fp.nch;          // last pixel a tile's window segment touches + 1
@@ -308,7 +371,8 @@ bool MixedInferenceCore::init(std::string& err) {
         int readers = 0;
         for (auto* L : graph.sorted) {
             if (L->fusedAway || L->isInputLayer) continue;
-            const bool reads = std::find(L->inputs.begin(), L->inputs.end(), t) != L->inputs.end() || L->residual == t;
+            const bool reads = std::find(L->inputs.begin(), L->inputs.end(), t) != L->inputs.end() || L->residual == t ||
+                               (L->typeName == "Conv2D" && static_cast<Conv2DLayer*>(L)->shortcutIn == t);
             if (!reads) continue;
             ++readers;
             only = only && L->typeName == "Conv2D" && static_cast<Conv2DLayer*>(L)->feedInput && L->inputs.size() >= 1 && L->inputs[0] == t && L->residual != t &&
@@ -645,6 +709,9 @@ int MixedInferenceCore::wait(int ticket) {
 int MixedInferenceCore::layerOutput(int layerId, float* host, size_t capacityFloats) {
     SNNB_REQUIRE(layerId >= 0 && layerId < (int) layers.size() && host, "layerOutput: bad argument");
     GenericModelLayer* L = layers[layerId].get();
+    SNNB_REQUIRE(!(L->typeName == "Conv2D" && static_cast<Conv2DLayer*>(L)->foldedInto),
+                 "layerOutput: layer %d (%s) was fused into the K loop of the convolution it is added to; load the model with fuse=0 to observe it", layerId,
+                 L->name.c_str());
     SNNB_REQUIRE(L->output, "layerOutput: layer %d (%s) has no device tensor", layerId, L->name.c_str());
     SNNB_REQUIRE(!(L->typeName == "Conv2D" && static_cast<Conv2DLayer*>(L)->fusedAct >= 0),
                  "layerOutput: layer %d (%s) was fused into its Add; load the model with fuse=0 to observe it", layerId, L->name.c_str());

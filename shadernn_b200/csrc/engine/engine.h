@@ -175,6 +175,11 @@ public:
     // Stride-2 stem with <= 4 input channels reading a model input: the input tensor carries a compact 4-channel copy
     // (snnb_tensor::feed_hi) and the weights get the matching K order (FeedPlan, kernels_umma.cu conv_rowwin_kernel feed mode).
     bool feedInput = false;
+    // Projection shortcut folded into this convolution's K loop (fusion pass in MixedInferenceCore::init): `shortcut` is the 1x1 conv
+    // whose product this layer adds, reading `shortcutIn`; the shortcut layer itself launches nothing and points back via `foldedInto`.
+    Conv2DLayer* shortcut    = nullptr;
+    Conv2DLayer* foldedInto  = nullptr;
+    snnb_tensor* shortcutIn  = nullptr;
     bool wantsPrepad(const snnb_tensor* in, const snnb_tensor* out, int convAlgo, int& ph, int& pw) const;
     Transform getOutputScaleDimAdjustment() const override; // conv2d.cpp:102-113
     void getOutputDims(uint32_t& w, uint32_t& h, uint32_t& d) const override;

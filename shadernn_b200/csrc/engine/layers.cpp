@@ -67,6 +67,7 @@ static const float* bnv(const std::map<std::string, std::vector<float>>& bn, con
     return (it == bn.end() || it->second.empty()) ? nullptr : it->second.data();
 }
 void Conv2DLayer::packWeights(PackedHost& p) {
+    if (foldedInto) return; // packed as the extra columns of the convolution it was folded into (which frees the host copy)
     const auto& bn = _desc.batchNormalization;
     const bool use = _desc.useBatchNormalization;
     pack_conv2d_host((int) numInputPlanes, (int) numOutputPlanes, (int) _desc.kernelSize, _desc.weights.data(), _desc.biases.empty() ? nullptr : _desc.biases.data(),
@@ -83,6 +84,14 @@ void Conv2DLayer::packWeights(PackedHost& p) {
         } else {
             pack_rowwin_host(p, (int) _desc.stride, 0);
         }
+    }
+    if (shortcut) {
+        const auto& sd = shortcut->_desc;
+        const bool sbn = sd.useBatchNormalization;
+        pack_shortcut_host((int) shortcut->numInputPlanes, sd.weights.data(), sd.biases.empty() ? nullptr : sd.biases.data(),
+                           sbn ? bnv(sd.batchNormalization, "gamma") : nullptr, sbn ? bnv(sd.batchNormalization, "beta") : nullptr,
+                           sbn ? bnv(sd.batchNormalization, "movingMean") : nullptr, sbn ? bnv(sd.batchNormalization, "movingVariance") : nullptr, p);
+        std::vector<float>().swap(shortcut->_desc.weights);
     }
     std::vector<float>().swap(_desc.weights); // host copy no longer needed
 }
@@ -118,8 +127,13 @@ int Conv2DLayer::run(snnb_context* ctx, const ExecOptions& opt) {
     a.act      = fusedAct >= 0 ? fusedAct : _desc.activation.id;
     a.alpha    = fusedAct >= 0 ? fusedAlpha : _desc.activation.alpha;
     a.precision = opt.precision;
+    a.shortcut = shortcutIn, a.sc_stride = shortcut ? (int) shortcut->_desc.stride : 1;
     const int want = algo != SNNB_ALGO_AUTO ? algo : opt.convAlgo;
     if (want != SNNB_ALGO_SIMT && conv2d_umma_supported(a)) return launch_conv2d_umma(ctx, a);
+    if (shortcut) {
+        set_error("%s: a folded projection shortcut runs on the tensor-core kernel only; load the model with fuse=0 for another algorithm", name.c_str());
+        return 2;
+    }
     if (want == SNNB_ALGO_TCGEN05) {
         set_error("%s: tcgen05 path requested but unsupported for this shape", name.c_str());
         return 2;

@@ -101,6 +101,10 @@ struct UmmaParams {
     int sk, sk_dp, sk_ctas;
     long long sk_units;
     int b_stages, b_stage_bytes; // halo mode: depth and stage size of the weight ring (3 x 32 KB, or 6 x 16 KB when a stage fits)
+    // Folded projection shortcut (plain mode only, ConvArgs::shortcut): a 1x1 stride-sc_stride convolution of another tensor onto the
+    // same output grid, computed as sc_cblocks extra K blocks after the k x k taps (operand tmS_hi / tmS_lo, weight columns
+    // ksize * ksize * ICp + cb * 64). sc_cblocks = 0: no shortcut.
+    int sc_cblocks, sc_stride;
 };
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -578,6 +582,38 @@ __host__ __device__ __forceinline__ int sk_first_work(const UmmaParams& p, int c
     return cta < p.sk_ctas ? p.sk_dp + 4 * cta : (cta < p.sk_dp ? cta : end);
 }
 
+// K block kb of a plain-mode launch: the k x k taps of the input come first, (tap, 64-channel block) in order kb = tap * cblocks + cb;
+// the sc_cblocks blocks of a folded shortcut follow. `wcol` is the block's first column in the packed weights.
+struct KBlock {
+    int sc, tap, cb, wcol;
+};
+__host__ __device__ __forceinline__ KBlock decode_kblock(const UmmaParams& p, int kb) {
+    const int kb_main = p.ksize * p.ksize * p.cblocks;
+    KBlock k;
+    k.sc  = kb >= kb_main;
+    k.tap = k.sc ? 0 : kb / p.cblocks;
+    k.cb  = k.sc ? kb - kb_main : kb - k.tap * p.cblocks;
+    k.wcol = (k.sc ? p.ksize * p.ksize : k.tap) * p.ICp + k.cb * UM_BLOCK_K;
+    return k;
+}
+// The producer's walk over K blocks [kb0, kb1): decoded once, then stepped (no divisions per K block). f(kb, sc, cb, kx, ky, wcol).
+// A range may straddle the end of the taps (split-K / stream-K pieces); the walk then switches to the shortcut operand once.
+template <class F> __host__ __device__ __forceinline__ void for_each_kblock(const UmmaParams& p, int kb0, int kb1, F&& f) {
+    const int ks = p.ksize, cbs = p.cblocks, icp = p.ICp, kb_main = ks * ks * cbs;
+    const KBlock k0 = decode_kblock(p, kb0);
+    int cb = k0.cb, kx = k0.tap % ks, ky = k0.tap / ks;
+    int wk = k0.wcol - k0.cb * UM_BLOCK_K; // tap * ICp; past the taps: ks * ks * ICp, the shortcut's first column
+    int kb = kb0;
+    for (const int e = kb1 < kb_main ? kb1 : kb_main; kb < e; ++kb) {
+        f(kb, false, cb, kx, ky, wk + cb * UM_BLOCK_K);
+        if (++cb == cbs) {
+            cb = 0, wk += icp;
+            if (++kx == ks) kx = 0, ++ky;
+        }
+    }
+    for (; kb < kb1; ++kb, ++cb) f(kb, true, cb, 0, 0, wk + cb * UM_BLOCK_K);
+}
+
 #define UM_TRACE(role, idx)                                                                          \
     do {                                                                                             \
         if (p.trace && blockIdx.x == 0 && lane == 0 && (idx) < 256) p.trace[(role) * 256 + (idx)] = clock64(); \
@@ -597,7 +633,7 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
                  const __grid_constant__ CUtensorMap tmB_lo, const __grid_constant__ CUtensorMap tmO_hi64, const __grid_constant__ CUtensorMap tmO_lo64,
                  const __grid_constant__ CUtensorMap tmO_hiT, const __grid_constant__ CUtensorMap tmO_loT, const __grid_constant__ CUtensorMap tmR_hi64,
                  const __grid_constant__ CUtensorMap tmR_lo64, const __grid_constant__ CUtensorMap tmR_hiT, const __grid_constant__ CUtensorMap tmR_loT,
-                 const UmmaParams p) {
+                 const __grid_constant__ CUtensorMap tmS_hi, const __grid_constant__ CUtensorMap tmS_lo, const UmmaParams p) {
     extern __shared__ uint8_t smem_raw[];
     constexpr bool ONE_BLOCK = TERMS != 3 || SPLIT_EPI; // the accumulator is one column block of n_blk (else [hi.hi + lo.hi | hi.lo])
     constexpr int EPI_TERMS  = ONE_BLOCK ? 2 : 3;       // what the epilogue templates need to know: one block or two
@@ -671,7 +707,7 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
     // The WEIGHTS of this CTA's first work item do not depend on the previous kernel: their loads go out before the dependency wait
     // (plain mode: the first K block's; halo mode: the first three taps'), so only the activations' latency is left after it.
     const int pre_total_tiles = p.tiles_x * p.tiles_y * p.tiles_n * p.tiles_oc;
-    const int pre_num_kb      = p.ksize * p.ksize * p.cblocks;
+    const int pre_num_kb      = p.ksize * p.ksize * p.cblocks + p.sc_cblocks;
     const int pre_end         = SK ? p.sk_dp + 4 * p.sk_ctas : pre_total_tiles * p.ksplit; // one past the last work id
     const int first_work      = SK ? sk_first_work(p, (int) blockIdx.x, pre_end) : (int) blockIdx.x;
     const bool pre_b          = (p.ablate & (2 | 16)) == 0 && first_work < pre_end; // ablate 16: no early weight loads (results stay correct)
@@ -688,14 +724,17 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
                 if (TERMS == 3) tma_load_2d(sB + b_lo_off, &tmB_lo, fb, tap * p.ICp, oc0);
             }
         } else {
-            const int kb0 = w0.kb0, cb = kb0 % p.cblocks, tap0 = kb0 / p.cblocks;
+            const int wcol    = decode_kblock(p, w0.kb0).wcol;
             const uint32_t fb = full_bar(0);
             mbar_expect_tx(fb, (TERMS == 1 ? 1u : 2u) * (uint32_t) p.rows_used * 128u + (TERMS == 3 ? 2u : 1u) * (uint32_t) p.n_blk * 128u);
-            tma_load_2d(smem_base + 2 * UM_A_BYTES, &tmB_hi, fb, tap0 * p.ICp + cb * UM_BLOCK_K, oc0);
-            if (TERMS == 3) tma_load_2d(smem_base + 2 * UM_A_BYTES + b_lo_off, &tmB_lo, fb, tap0 * p.ICp + cb * UM_BLOCK_K, oc0);
+            tma_load_2d(smem_base + 2 * UM_A_BYTES, &tmB_hi, fb, wcol, oc0);
+            if (TERMS == 3) tma_load_2d(smem_base + 2 * UM_A_BYTES + b_lo_off, &tmB_lo, fb, wcol, oc0);
         }
     }
-    pdl_wait(); // everything above (barriers, TMEM, tensor-map prefetch, first weights) overlapped with the previous kernel's tail
+    // everything above (barriers, TMEM, tensor-map prefetch, first weights) overlapped with the previous kernel's tail. A folded
+    // shortcut's operand was written two launches back, not by the previous grid: that grid itself passed this wait on ITS
+    // predecessor before it could complete, so once it has completed every earlier grid has too.
+    pdl_wait();
     if (warp == 0) UM_TRACE(5, 0); // kernel entry (after the dependency wait)
     if (p.trace && threadIdx.x == 0) { // wall-clock (ns) envelope over ALL CTAs: [5][8] = earliest entry, [5][9] = latest exit, [5][10..11] CTA 0's own
         unsigned long long g;
@@ -708,7 +747,7 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
 
     const int m_tiles     = p.tiles_x * p.tiles_y * p.tiles_n;
     const int total_tiles = m_tiles * p.tiles_oc;
-    const int num_kb      = p.ksize * p.ksize * p.cblocks;
+    const int num_kb      = p.ksize * p.ksize * p.cblocks + p.sc_cblocks;
     const int total_work  = SK ? p.sk_dp + 4 * p.sk_ctas : total_tiles * p.ksplit; // work item = (tile, K range); one past the last work id
 
     if (warp == 0) {
@@ -718,7 +757,7 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
             uint32_t phase = 0, hphase = 0;
             (void) hstage, (void) hphase;
             const uint32_t tx_bytes = (TERMS == 1 ? 1u : 2u) * (uint32_t) p.rows_used * 128u + (TERMS == 3 ? 2u : 1u) * (uint32_t) p.n_blk * 128u;
-            const int ks = p.ksize, cbs = p.cblocks, icp = p.ICp;
+            const int cbs = p.cblocks, icp = p.ICp;
             const bool skip_tma = (p.ablate & 2) != 0;
             const uint32_t b_lo_off = (uint32_t) p.n_blk * 128u; // B_lo rows follow B_hi's: one [2 n_blk x 64] operand
             int tr = 0;
@@ -757,7 +796,8 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
                 const int kb0 = wi.kb0, kb1 = wi.kb1;
                 // Keep this loop lean: it runs once per K block and every stall here delays the whole pipeline (no divisions,
                 // no parameter loads: ncu r01 showed ~60 dependent scalar instructions/iteration bounding the kernel).
-                // K block kb = (ky * ks + kx) * cbs + cb; the counters are decoded once per work item and then stepped.
+                // K block kb = (ky * ks + kx) * cbs + cb, then a folded shortcut's blocks; the counters are decoded once per work item
+                // and then stepped (for_each_kblock).
                 if constexpr (HALO) {
                     // K order (cb, tap): one halo tile per channel block, then the nine taps' weights. The halo tile of the NEXT
                     // unit (next channel block, or the next work item's first) is requested one unit ahead, after this unit's first
@@ -818,10 +858,9 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
                     work = nwork;
                     continue;
                 }
-                int cb = kb0 % cbs, tap0 = kb0 / cbs;
-                int kx = tap0 % ks, ky = tap0 / ks;
-                int wk = tap0 * icp; // K coordinate into the packed weights = tap * ICp + cb * 64
-                for (int kb = kb0; kb < kb1; ++kb) {
+                // the folded shortcut's box: the same output pixels at its own stride, pad 0 (a 1x1 convolution)
+                const int sx0 = bx * p.tw * p.sc_stride, sy0 = by * p.th * p.sc_stride;
+                for_each_kblock(p, kb0, kb1, [&](int kb, bool sc, int cb, int kx, int ky, int wcol) {
                     mbar_wait(empty_bar(stage), phase ^ 1u);
                     UM_TRACE(0, tr);
                     ++tr;
@@ -832,20 +871,19 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
                         } else {
                             const bool pre = seq == 0 && kb == kb0 && pre_b; // expect_tx + the weights went out before the dependency wait
                             if (!pre) mbar_expect_tx(fb, tx_bytes);
-                            tma_load_4d(sA, &tmA_hi, fb, cb * UM_BLOCK_K, ix0 + kx, iy0 + ky, n0);
-                            if (TERMS >= 2) tma_load_4d(sA + UM_A_BYTES, &tmA_lo, fb, cb * UM_BLOCK_K, ix0 + kx, iy0 + ky, n0);
+                            const CUtensorMap* a_hi = sc ? &tmS_hi : &tmA_hi;
+                            const CUtensorMap* a_lo = sc ? &tmS_lo : &tmA_lo;
+                            const int ax = sc ? sx0 : ix0 + kx, ay = sc ? sy0 : iy0 + ky;
+                            tma_load_4d(sA, a_hi, fb, cb * UM_BLOCK_K, ax, ay, n0);
+                            if (TERMS >= 2) tma_load_4d(sA + UM_A_BYTES, a_lo, fb, cb * UM_BLOCK_K, ax, ay, n0);
                             if (!pre) {
-                                tma_load_2d(sA + 2 * UM_A_BYTES, &tmB_hi, fb, wk + cb * UM_BLOCK_K, oc0);
-                                if (TERMS == 3) tma_load_2d(sA + 2 * UM_A_BYTES + b_lo_off, &tmB_lo, fb, wk + cb * UM_BLOCK_K, oc0);
+                                tma_load_2d(sA + 2 * UM_A_BYTES, &tmB_hi, fb, wcol, oc0);
+                                if (TERMS == 3) tma_load_2d(sA + 2 * UM_A_BYTES + b_lo_off, &tmB_lo, fb, wcol, oc0);
                             }
                         }
                     }
                     if (++stage == STAGES) stage = 0, phase ^= 1u;
-                    if (++cb == cbs) {
-                        cb = 0, wk += icp;
-                        if (++kx == ks) kx = 0, ++ky;
-                    }
-                }
+                });
                 work = take_next();
             }
         }
@@ -1675,6 +1713,30 @@ bool conv2d_umma_supported(const ConvArgs& a) {
     return true;
 }
 
+// halo mode (3x3, stride 1): 8 x 16-pixel tiles whose nine taps share one halo load; taken when the cost model prefers it to the plain
+// plan of cost `plain_cost` (fewer bytes per K block against the MMA rows lost where 8 / 16 do not divide the feature map)
+static bool halo_plan(const snnb_context* ctx, const ConvArgs& a, int cblocks, int terms, double plain_cost, OcPlan& hp) {
+    static const bool no_halo = getenv("SNNB_NO_HALO") != nullptr;
+    if (no_halo || a.k != 3 || a.stride != 1 || a.pad_x > 1 || a.pad_y > 1) return false;
+    const int hx = (a.out->w + HL_TW - 1) / HL_TW, hy = (a.out->h + HL_TH - 1) / HL_TH;
+    hp = plan_oc_ksplit(a.out->c, hx * hy * a.out->n, UM_BLOCK_M, HL_TW, 9 * cblocks, ctx->sm_count, terms, true);
+    return hp.n_blk > 0 && hp.cost < plain_cost;
+}
+
+bool conv2d_umma_fold_supported(const snnb_context* ctx, const ConvArgs& a) {
+    if (!a.shortcut || a.residual || !conv2d_umma_supported(a) || rowwin_supported(a)) return false;
+    // stride <= 2 keeps the shortcut's box (tw * s, th * s with tw, th <= 128) within TMA's 256 elements per dimension
+    if (!(a.sc_stride == 1 || a.sc_stride == 2) || a.shortcut->n != a.out->n || !a.shortcut->lo != !a.in->lo) return false;
+    const TilePlan tp = plan_tiles(a.out->n, a.out->h, a.out->w, a.stride);
+    if (tp.tw <= 0) return false;
+    // the layer as it would run unfolded: a layer the halo mode serves better keeps its own launch (the fold is plain mode only)
+    const int cblocks = (a.in->c + UM_BLOCK_K - 1) / UM_BLOCK_K, terms = conv_terms(ctx, a);
+    const OcPlan op   = plan_oc_ksplit(a.out->c, tp.tiles_x * tp.tiles_y * tp.tiles_n, tp.tw * tp.th * tp.tn, tp.tw, a.k * a.k * cblocks, ctx->sm_count, terms, false,
+                                       a.stream_k);
+    OcPlan hp;
+    return op.n_blk > 0 && !halo_plan(ctx, a, cblocks, terms, op.cost, hp);
+}
+
 enum { ATTR_UMMA = 1u, ATTR_ROWWIN = 2u, ATTR_DW1 = 4u, ATTR_DW2 = 8u }; // bits of snnb_context::func_attr_mask
 
 typedef void (*RowWinKernel)(const CUtensorMap, const CUtensorMap, const CUtensorMap, const CUtensorMap, const CUtensorMap, const CUtensorMap, const CUtensorMap,
@@ -1801,8 +1863,14 @@ static int launch_conv2d_rowwin(snnb_context* ctx, const ConvArgs& a, EncodeTile
 int launch_conv2d_umma(snnb_context* ctx, const ConvArgs& a) {
     EncodeTiledFn encode = get_encode(ctx);
     SNNB_REQUIRE(encode, "launch_conv2d_umma: cuTensorMapEncodeTiled is unavailable in this driver");
-    if (rowwin_supported(a)) return launch_conv2d_rowwin(ctx, a, encode);
-    SNNB_REQUIRE(!a.in->feed_only, "launch_conv2d_umma: the input tensor only exists as a stem feed, which this launch cannot read");
+    if (rowwin_supported(a)) {
+        SNNB_REQUIRE(!a.shortcut, "launch_conv2d_umma: a folded shortcut needs the plain tensor-core kernel, not the row-window kernel");
+        return launch_conv2d_rowwin(ctx, a, encode);
+    }
+    SNNB_REQUIRE(!a.in->feed_only && !(a.shortcut && a.shortcut->feed_only), "launch_conv2d_umma: the input tensor only exists as a stem feed, which this launch cannot read");
+    SNNB_REQUIRE(!(a.shortcut && a.residual), "launch_conv2d_umma: a folded shortcut and a residual operand are exclusive");
+    SNNB_REQUIRE(!a.shortcut || ((a.sc_stride == 1 || a.sc_stride == 2) && a.shortcut->n == a.out->n), "launch_conv2d_umma: unsupported shortcut (stride %d)",
+                 a.sc_stride);
     const snnb_tensor* in = a.in;
     snnb_tensor* out      = a.out;
     UmmaParams p;
@@ -1817,24 +1885,20 @@ int launch_conv2d_umma(snnb_context* ctx, const ConvArgs& a) {
     p.tiles_x = tp.tiles_x, p.tiles_y = tp.tiles_y, p.tiles_n = tp.tiles_n;
     p.ksize = a.k, p.stride = a.stride, p.pad_x = a.pad_x, p.pad_y = a.pad_y;
     p.cblocks = (in->c + UM_BLOCK_K - 1) / UM_BLOCK_K;
+    p.sc_cblocks = a.shortcut ? (a.shortcut->c + UM_BLOCK_K - 1) / UM_BLOCK_K : 0, p.sc_stride = a.shortcut ? a.sc_stride : 1;
+    const int num_kb = a.k * a.k * p.cblocks + p.sc_cblocks;
     const int terms = conv_terms(ctx, a);
     p.has_lo        = out->lo != nullptr;
     p.b_stages = 0, p.b_stage_bytes = 0;
-    OcPlan op       = plan_oc_ksplit(out->c, tp.tiles_x * tp.tiles_y * tp.tiles_n, p.rows_used, tp.tw, a.k * a.k * p.cblocks, ctx->sm_count, terms, false, a.stream_k);
-    // halo mode (3x3, stride 1): 8 x 16-pixel tiles whose nine taps share one halo load; taken when the cost model prefers it
-    // (fewer bytes per K block against the MMA rows lost where 8 / 16 do not divide the feature map)
-    static const bool no_halo = getenv("SNNB_NO_HALO") != nullptr;
-    bool halo                 = false;
-    if (!no_halo && a.k == 3 && a.stride == 1 && a.pad_x <= 1 && a.pad_y <= 1) {
-        const int hx = (out->w + HL_TW - 1) / HL_TW, hy = (out->h + HL_TH - 1) / HL_TH;
-        const OcPlan hp = plan_oc_ksplit(out->c, hx * hy * out->n, UM_BLOCK_M, HL_TW, 9 * p.cblocks, ctx->sm_count, terms, true);
-        if (hp.n_blk > 0 && hp.cost < op.cost) {
-            halo = true, op = hp;
-            p.b_stage_bytes = (terms == 3 ? 2 : 1) * op.n_blk * 128 <= UM_B_BYTES ? UM_B_BYTES : 2 * UM_B_BYTES; // 16 KB when a stage fits, else 32 KB
-            p.b_stages      = HL_B_RING_BYTES / p.b_stage_bytes;
-            p.tw = HL_TW, p.th = HL_TH, p.tn = 1, p.rows_used = UM_BLOCK_M;
-            p.tiles_x = hx, p.tiles_y = hy, p.tiles_n = out->n;
-        }
+    OcPlan op       = plan_oc_ksplit(out->c, tp.tiles_x * tp.tiles_y * tp.tiles_n, p.rows_used, tp.tw, num_kb, ctx->sm_count, terms, false, a.stream_k);
+    OcPlan hp;
+    const bool halo = !a.shortcut && halo_plan(ctx, a, p.cblocks, terms, op.cost, hp); // the halo producer has no shortcut operand
+    if (halo) {
+        op              = hp;
+        p.b_stage_bytes = (terms == 3 ? 2 : 1) * op.n_blk * 128 <= UM_B_BYTES ? UM_B_BYTES : 2 * UM_B_BYTES; // 16 KB when a stage fits, else 32 KB
+        p.b_stages      = HL_B_RING_BYTES / p.b_stage_bytes;
+        p.tw = HL_TW, p.th = HL_TH, p.tn = 1, p.rows_used = UM_BLOCK_M;
+        p.tiles_x = (out->w + HL_TW - 1) / HL_TW, p.tiles_y = (out->h + HL_TH - 1) / HL_TH, p.tiles_n = out->n;
     }
     SNNB_REQUIRE(op.n_blk > 0, "launch_conv2d_umma: no output-channel plan");
     p.n_blk = op.n_blk, p.tiles_oc = op.tiles_oc, p.ksplit = op.ksplit, p.kb_per_split = op.kb_per_split;
@@ -1866,21 +1930,30 @@ int launch_conv2d_umma(snnb_context* ctx, const ConvArgs& a) {
     p.act = a.act, p.alpha = a.alpha;
     static const int ablate = getenv("SNNB_UMMA_ABLATE") ? atoi(getenv("SNNB_UMMA_ABLATE")) : 0;
     p.ablate                = ablate;
-    SNNB_REQUIRE(a.w->kp == a.k * a.k * p.ICp, "launch_conv2d_umma: packed weights do not match (kp %d vs %d)", a.w->kp, a.k * a.k * p.ICp);
+    const int kp_want = a.k * a.k * p.ICp + (a.shortcut ? round_up(a.shortcut->c, 8) : 0); // [taps | shortcut] columns
+    SNNB_REQUIRE(a.w->kp == kp_want, "launch_conv2d_umma: packed weights do not match (kp %d vs %d)", a.w->kp, kp_want);
 
-    CUtensorMap tmA[2], tmB[2];
-    {
-        const cuuint64_t dims[4]    = {(cuuint64_t) in->c, (cuuint64_t) in->w, (cuuint64_t) in->h, (cuuint64_t) in->n};
-        const cuuint64_t strides[3] = {(cuuint64_t) in->cp * 2, (cuuint64_t) in->w * in->cp * 2, (cuuint64_t) in->h * in->w * in->cp * 2};
-        const cuuint32_t box[4]     = {(cuuint32_t) UM_BLOCK_K, (cuuint32_t) (halo ? HL_W : p.tw * a.stride), (cuuint32_t) (halo ? HL_H : p.th * a.stride), (cuuint32_t) p.tn};
-        const cuuint32_t estr[4]    = {1, (cuuint32_t) a.stride, (cuuint32_t) a.stride, 1};
-        __half* planes[2]    = {in->hi, in->lo ? in->lo : in->hi}; // fp16 storage mode: the lo map is never issued
+    // A operand maps: box = the output tile's pixels at traversal stride s (halo mode: the halo tile); channel tail zero-filled
+    auto encode_a = [&](const snnb_tensor* t, int s, int bw, int bh, CUtensorMap (&maps)[2]) {
+        const cuuint64_t dims[4]    = {(cuuint64_t) t->c, (cuuint64_t) t->w, (cuuint64_t) t->h, (cuuint64_t) t->n};
+        const cuuint64_t strides[3] = {(cuuint64_t) t->cp * 2, (cuuint64_t) t->w * t->cp * 2, (cuuint64_t) t->h * t->w * t->cp * 2};
+        const cuuint32_t box[4]     = {(cuuint32_t) UM_BLOCK_K, (cuuint32_t) bw, (cuuint32_t) bh, (cuuint32_t) p.tn};
+        const cuuint32_t estr[4]    = {1, (cuuint32_t) s, (cuuint32_t) s, 1};
+        __half* planes[2]    = {t->hi, t->lo ? t->lo : t->hi}; // fp16 storage mode: the lo map is never issued
         for (int i = 0; i < 2; ++i) {
-            CUresult r = encode(&tmA[i], CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, planes[i], dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+            CUresult r = encode(&maps[i], CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, planes[i], dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                                 CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-            SNNB_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled(A) failed: %d (dims %d %d %d %d box %u %u %u %u)", (int) r, in->c, in->w, in->h, in->n, box[0],
+            SNNB_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled(A) failed: %d (dims %d %d %d %d box %u %u %u %u)", (int) r, t->c, t->w, t->h, t->n, box[0],
                          box[1], box[2], box[3]);
         }
+        return 0;
+    };
+    CUtensorMap tmA[2], tmB[2], tmS[2];
+    if (encode_a(in, a.stride, halo ? HL_W : p.tw * a.stride, halo ? HL_H : p.th * a.stride, tmA)) return 2;
+    if (!a.shortcut) {
+        tmS[0] = tmA[0], tmS[1] = tmA[1]; // never issued
+    } else if (encode_a(a.shortcut, a.sc_stride, p.tw * a.sc_stride, p.th * a.sc_stride, tmS)) {
+        return 2;
     }
     {
         const cuuint64_t dims[2]    = {(cuuint64_t) a.w->kp, (cuuint64_t) a.w->ocr};
@@ -1923,7 +1996,7 @@ int launch_conv2d_umma(snnb_context* ctx, const ConvArgs& a) {
     const int grid        = p.sk ? (p.sk_dp > 0 ? ctx->sm_count : p.sk_ctas) : std::min(total_tiles * p.ksplit, ctx->sm_count);
     // short K loop (1x1 convolutions): the layer runs at the speed of the epilogue -> two independent epilogue groups
     static const bool no_split_epi = getenv("SNNB_NO_SPLIT_EPI") != nullptr;
-    const bool split_epi           = !halo && !no_split_epi && !p.sk && p.ksplit == 1 && p.ksize * p.ksize * p.cblocks <= 3 && total_tiles >= 2 * grid;
+    const bool split_epi           = !halo && !no_split_epi && !p.sk && p.ksplit == 1 && num_kb <= 3 && total_tiles >= 2 * grid;
     ctx->last_kernel = halo ? "conv_umma_kernel<halo>"
                             : (split_epi ? "conv_umma_kernel<short-K>" : (p.sk ? "conv_umma_kernel<stream-K>" : (p.ksplit > 1 ? "conv_umma_kernel<split-K>" : "conv_umma_kernel")));
     p.trace = nullptr;
@@ -1935,15 +2008,15 @@ int launch_conv2d_umma(snnb_context* ctx, const ConvArgs& a) {
     auto* k_halo  = terms == 3 ? conv_umma_kernel<HL_B_STAGES, false, 3, true> : (terms == 2 ? conv_umma_kernel<HL_B_STAGES, false, 2, true> : conv_umma_kernel<HL_B_STAGES, false, 1, true>);
     const cudaError_t le =
         halo      ? launch_k_pdl(k_halo, dim3(grid), dim3(UM_THREADS), HL_SMEM_BYTES, ctx->stream, tmA[0], tmA[1], tmB[0], tmB[1], tmO64[0], tmO64[1], tmOT[0], tmOT[1], tmR64[0],
-                                 tmR64[1], tmRT[0], tmRT[1], p)
+                                 tmR64[1], tmRT[0], tmRT[1], tmS[0], tmS[1], p)
         : split_epi ? launch_k_pdl(k_split, dim3(grid), dim3(UM_THREADS), UM_SMEM_BYTES_SPLIT, ctx->stream, tmA[0], tmA[1], tmB[0], tmB[1], tmO64[0], tmO64[1], tmOT[0], tmOT[1],
-                                 tmR64[0], tmR64[1], tmRT[0], tmRT[1], p)
+                                 tmR64[0], tmR64[1], tmRT[0], tmRT[1], tmS[0], tmS[1], p)
                   : launch_k_pdl(k_plain, dim3(grid), dim3(UM_THREADS), UM_SMEM_BYTES, ctx->stream, tmA[0], tmA[1], tmB[0], tmB[1], tmO64[0], tmO64[1], tmOT[0], tmOT[1], tmR64[0],
-                                 tmR64[1], tmRT[0], tmRT[1], p);
+                                 tmR64[1], tmRT[0], tmRT[1], tmS[0], tmS[1], p);
     if (p.trace) {
         char hdr[256];
         snprintf(hdr, sizeof hdr, "conv k%d s%d IC%d OC%d out %dx%dx%d n_blk %d tiles %d grid %d num_kb %d ksplit %d terms %d halo %d", a.k, a.stride, in->c, out->c, out->n,
-                 out->h, out->w, p.n_blk, total_tiles, grid, p.ksize * p.ksize * p.cblocks, split_epi ? -1 : (p.sk ? -2 : p.ksplit), terms, (int) halo); // ksplit -1 = split-epilogue variant, -2 = stream-K
+                 out->h, out->w, p.n_blk, total_tiles, grid, num_kb, split_epi ? -1 : (p.sk ? -2 : p.ksplit), terms, (int) halo); // ksplit -1 = split-epilogue variant, -2 = stream-K
         if (trace_end(ctx, p.trace, hdr)) return 1;
     }
     cudaError_t e = le != cudaSuccess ? le : cudaGetLastError();
@@ -2207,6 +2280,45 @@ int streamk_schedule(int tiles, int num_kb, int sms, int* rows, int capacity) {
             ++n;
         }
     return n;
+}
+
+// Every K block the producer loads, per work item, for a launch of `tiles` tiles with ksize x ksize taps over `cblocks` channel blocks
+// (channel pitch icp) and a folded shortcut of sc_cblocks blocks: split-K into `ksplit` ranges, or stream-K over `sms` CTAs when
+// ksplit == 0. The work items come from decode_work, the blocks from for_each_kblock - the functions the kernel's roles call. One row
+// {tile, kb, sc, tap, cb, wcol} per K block. Returns the number of rows, or -1 for arguments no launch has (or nothing to cut for stream-K).
+int kblock_schedule(int ksize, int cblocks, int icp, int sc_cblocks, int tiles, int ksplit, int sms, int* rows, int capacity) {
+    if (ksize < 1 || cblocks < 1 || icp < 8 || sc_cblocks < 0 || tiles < 1 || ksplit < 0 || sms < 1) return -1;
+    UmmaParams p {};
+    p.ksize = ksize, p.cblocks = cblocks, p.ICp = icp, p.sc_cblocks = sc_cblocks, p.sc_stride = 1;
+    const int num_kb = ksize * ksize * cblocks + sc_cblocks;
+    std::vector<WorkItem> items;
+    if (ksplit > 0) {
+        p.ksplit = ksplit, p.kb_per_split = (num_kb + ksplit - 1) / ksplit;
+        for (int work = 0; work < tiles * ksplit; ++work) items.push_back(decode_work<false>(p, work, tiles, num_kb));
+    } else {
+        int dp = 0, ctas = 0;
+        long long units = 0;
+        if (tiles % sms == 0 || !streamk_split(tiles, num_kb, sms, dp, units, ctas)) return -1;
+        p.sk = 1, p.sk_dp = dp, p.sk_ctas = ctas, p.sk_units = units, p.ksplit = 1, p.kb_per_split = num_kb;
+        const int grid = dp > 0 ? sms : ctas, end = dp + 4 * ctas;
+        for (int cta = 0; cta < grid; ++cta)
+            for (int work = sk_first_work(p, cta, end); work < end; work = sk_next_work(p, work, cta, grid, num_kb, end)) items.push_back(decode_work<true>(p, work, tiles, num_kb));
+    }
+    struct Row { // for_each_kblock is __host__ __device__: a functor with a callable of the same kind, not a host lambda
+        int *rows, capacity, ksize, tile, n;
+        __host__ __device__ void operator()(int kb, bool sc, int cb, int kx, int ky, int wcol) {
+            if (n < capacity) {
+                int* r = rows + 6 * (size_t) n;
+                r[0] = tile, r[1] = kb, r[2] = sc, r[3] = ky * ksize + kx, r[4] = cb, r[5] = wcol;
+            }
+            ++n;
+        }
+    } row {rows, capacity, ksize, 0, 0};
+    for (const WorkItem& w : items) {
+        row.tile = w.tile;
+        for_each_kblock(p, w.kb0, w.kb1, row);
+    }
+    return row.n;
 }
 
 } // namespace snnb

@@ -81,6 +81,31 @@ void pack_conv2d_host(int IC, int OC, int k, const float* w_oihw, const float* b
     }
 }
 
+void pack_shortcut_host(int IC, const float* w_oi, const float* bias, const float* g, const float* b, const float* m, const float* v, PackedHost& out) {
+    const int OC = out.out_ch;
+    std::vector<float> scale, shift;
+    bn_fold(OC, bias, g, b, m, v, scale, shift);
+    // [OCr][kp] -> [OCr][kp + ICp]: the shortcut's columns follow the taps', in the order the producer walks its K blocks
+    const int kp = out.kp + round_up(IC, 8);
+    std::vector<__half> hi((size_t) out.ocr * kp, __float2half_rn(0.0f)), lo((size_t) out.ocr * kp, __float2half_rn(0.0f));
+    for (int o = 0; o < out.ocr; ++o) {
+        std::memcpy(&hi[(size_t) o * kp], &out.w_hi[(size_t) o * out.kp], out.kp * sizeof(__half));
+        std::memcpy(&lo[(size_t) o * kp], &out.w_lo[(size_t) o * out.kp], out.kp * sizeof(__half));
+    }
+    for (int o = 0; o < OC; ++o) {
+        out.bias[o] += shift[o];
+        for (int i = 0; i < IC; ++i) {
+            const float wv  = w_oi[(size_t) o * IC + i] * scale[o];
+            const __half h  = __float2half_rn(wv);
+            const size_t at = (size_t) o * kp + out.kp + i;
+            hi[at] = h;
+            lo[at] = __float2half_rn(wv - __half2float(h));
+        }
+    }
+    out.w_hi.swap(hi), out.w_lo.swap(lo);
+    out.kp = kp;
+}
+
 void pack_rowwin_host(PackedHost& p, int stride, int pad_x) {
     RowPlan rp;
     if (p.kind != 1 || p.in_ch > 8 || p.out_ch > 64 || !make_row_plan(p.kernel, stride, pad_x, rp)) return;

@@ -188,10 +188,19 @@ struct ConvArgs {
     float alpha;
     int precision = -1; // SNNB_PRECISION_* of this launch; -1 = the context's default
     bool stream_k = false; // the planner may choose the stream-K decomposition (SNNB_ALGO_TCGEN05_STREAMK)
+    // Folded projection shortcut (tensor path only): out = conv(in) + conv1x1_stride(shortcut), the second product as extra K blocks
+    // of the same GEMM. The weights then carry [k*k*ICp | ICp_shortcut] columns and one summed bias; `residual` must be null.
+    const snnb_tensor* shortcut = nullptr;
+    int sc_stride = 1;
 };
 int launch_conv2d_simt(snnb_context* ctx, const ConvArgs& a);
 int launch_conv2d_umma(snnb_context* ctx, const ConvArgs& a); // kernels_umma.cu (tcgen05 + TMA)
 bool conv2d_umma_supported(const ConvArgs& a);
+// Would launch_conv2d_umma run `a` (shortcut set, weights may be a probe) in plain mode, the only mode that reads a shortcut? False for
+// the row-window kernel, for layers the planner gives to the halo mode, and for shortcuts the TMA box cannot express.
+bool conv2d_umma_fold_supported(const snnb_context* ctx, const ConvArgs& a);
+// host walk of every K block of a (folded) launch's work items, as the producer visits them (tests); see kernels_umma.cu
+int kblock_schedule(int ksize, int cblocks, int icp, int sc_cblocks, int tiles, int ksplit, int sms, int* rows, int capacity);
 int streamk_schedule(int tiles, int num_kb, int sms, int* rows, int capacity); // host evaluation of the stream-K work decomposition (tests)
 int launch_depthwise(snnb_context* ctx, const ConvArgs& a);
 bool depthwise_tma_supported(const ConvArgs& a);          // 3x3 stride 1/2: TMA-staged, register-tiled (kernels_umma.cu)
@@ -298,6 +307,9 @@ struct PackedHost {
 };
 void pack_conv2d_host(int IC, int OC, int k, const float* w_oihw, const float* bias, const float* g, const float* b, const float* m, const float* v,
                       PackedHost& out);
+// Appends a folded 1x1 projection shortcut (weights [OC][IC], bias and BatchNorm folded as in pack_conv2d_host) to the tensor-core
+// operand of an already packed convolution: w_hi/lo become [OCr][k*k*ICp + round_up(IC, 8)], the bias becomes the sum of both biases.
+void pack_shortcut_host(int IC, const float* w_oi, const float* bias, const float* g, const float* b, const float* m, const float* v, PackedHost& out);
 // Adds the row-window operand (w_row_hi/lo) for small-IC convolutions; needs the layer's stride and x padding.
 void pack_rowwin_host(PackedHost& p, int stride, int pad_x);
 // Adds the feed-mode operand (w_feed_hi/lo) when make_feed_plan() accepts the layer.
